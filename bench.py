@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- GCUPS of the adaptive-banded sequence-to-POA-graph DP hot path.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--groups G]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--groups G] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2], the one the metric is quoted on): synthetic read groups,
 50 reads x 10 kbp, 5 % ONT-like error, global alignment, convex gaps (-O 4,24 -E 2,1).
@@ -21,6 +21,9 @@ Printed JSON (rank 0):
   cpu_baseline  the UNMODIFIED reference (oracle/_ref/libabpoa_ref.so, AVX2) on the host cores,
             one process per physical core, on a bounded sample of the same groups.
 --impl reference prints the reference arm's line (CPU only; rank 0 alone runs).
+--dump-outputs DIR  (rank 0) writes what the last timed step returned to its caller as DIR/<name>.npy: per group the DP
+            cells, aligned reads and consensus length, and for a fixed sample of groups the consensus bases and their
+            coverage (see dump_outputs).  The inputs are seeded, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -42,6 +45,7 @@ ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
 
 METRIC = "GCUPS (DP cells/s), global/convex 10 kbp"
+REF_LIB = ROOT / "oracle" / "_ref" / "libabpoa_ref.so"      # the unmodified reference (oracle/Makefile builds it where its sources are)
 
 
 def physical_cores() -> int:
@@ -106,7 +110,7 @@ def _ref_worker(args):
     from abpoa_b200 import capi, synth
     from abpoa_b200.aligner import PoaSession
     w = synth.WORKLOADS[wname]
-    lib = capi.load_library(ROOT / "oracle" / "_ref" / "libabpoa_ref.so")     # the unmodified reference (oracle/Makefile)
+    lib = capi.load_library(REF_LIB)
     cells = 0
     reads_done = 0
     groups = [synth.make_group(seed, n_reads, length, w.err, w.cfg.m) for seed in seeds]     # outside the timed window
@@ -163,6 +167,38 @@ def cpu_baseline_block(wname: str, w, ref_groups: int, base_seed: int) -> tuple[
     return blk, a
 
 
+DUMP_SAMPLE_GROUPS = 256            # groups whose consensus and coverage are written by --dump-outputs (seeded choice)
+
+
+def dump_outputs(out_dir: str, results) -> None:
+    """The results of one step (BatchEngine.run_packed with keep_results=True), as .npy files under `out_dir`:
+    group_dp_cells, group_n_aligned, group_cons_len (float64, one per group), sample_groups (the sampled group
+    indices), sample_cons_offsets (float64, start of each sampled consensus in the concatenation, plus the end),
+    sample_cons_bases and sample_cons_cov (float32, the first consensus of each sampled group, concatenated)."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    n = len(results)
+    k = min(n, DUMP_SAMPLE_GROUPS)
+    sample = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False)) if n else np.zeros(0, dtype=np.int64)
+    first = lambda arrs: arrs[0] if arrs else np.zeros(0)
+    bases = [first(results[g].cons) for g in sample]
+    cov = [first(results[g].cov) for g in sample]
+    arrays = {
+        "group_dp_cells": np.array([r.dp_cells for r in results], dtype=np.float64),
+        "group_n_aligned": np.array([r.n_aligned for r in results], dtype=np.float64),
+        "group_cons_len": np.array([sum(len(c) for c in r.cons) for r in results], dtype=np.float64),
+        "sample_groups": sample.astype(np.float64),
+        "sample_cons_offsets": np.concatenate([[0], np.cumsum([len(b) for b in bases])]).astype(np.float64),
+        "sample_cons_bases": np.concatenate(bases).astype(np.float32) if bases else np.zeros(0, dtype=np.float32),
+        "sample_cons_cov": np.concatenate(cov).astype(np.float32) if cov else np.zeros(0, dtype=np.float32),
+    }
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"--dump-outputs would write {total} bytes"
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", a)
+
+
 # ------------------------------------------------------------------------------------------------
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons during the timed region (B200_PROFILING.md recipe)."""
@@ -206,7 +242,14 @@ def main():
     ap.add_argument("--groups", type=int, default=0, help="groups per GPU (default: the config's 1000)")
     ap.add_argument("--ref-groups", type=int, default=0, help="groups in one reference sample (default: one per core)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if not REF_LIB.exists():
+        if args.impl == "reference":
+            ap.error(f"{REF_LIB} is not built")
+        args.no_cpu_baseline = True          # the CPU baseline needs the reference library; the GPU measurement does not
     if args.warmup < 3:
         args.warmup = 3
 
@@ -303,14 +346,23 @@ def main():
     t0 = time.perf_counter()
     cells = 0
     cons_bases = 0
-    for _ in range(args.steps):
-        res = eng.run_packed(abpt, packed, keep_results=False)
+    last = None
+    for step in range(args.steps):
+        if args.dump_outputs and step == args.steps - 1:
+            # the last step also hands its consensus arrays back to the caller, to be written after the timed region
+            last = eng.run_packed(abpt, packed, keep_results=True)
+            res = [(r.dp_cells, r.n_aligned, sum(len(c) for c in r.cons)) for r in last]
+        else:
+            res = eng.run_packed(abpt, packed, keep_results=False)
         cells += sum(r[0] for r in res)
         cons_bases += sum(r[2] for r in res)
     barrier()
     elapsed = time.perf_counter() - t0
     clocks = sampler.stop() if rank == 0 else None
     st = eng.stats()
+    if last is not None and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+        last = None
     t = torch.tensor([elapsed, st["chain_device_ms"]], dtype=torch.float64, device="cuda")
     c = torch.tensor([float(cells), float(packed.total_reads * args.steps), float(st["launches"]), float(st["h2d_bytes"]), float(st["d2h_bytes"]),
                       float(st["chain_cells"]), float(st["chain_groups"]), float(st["chain_fallback_groups"]), st["chain_dp_ms"], st["chain_fuse_ms"],
@@ -328,7 +380,7 @@ def main():
     # engine, upload once, replay back to back with CUDA-event timing (per-launch numbers for the roofline)
     eng.run_packed(abpt, packed, keep_results=False, capture=True)
     barrier()
-    rp = eng.replay(abpt, warmup=1, repeats=max(args.steps, 2))
+    rp = eng.replay(abpt, warmup=1, repeats=args.steps)
     eng.clear_capture()
     kt = torch.tensor([rp["kernel_ms"]], dtype=torch.float64, device="cuda")
     kc = torch.tensor([float(rp["cells"])], dtype=torch.float64, device="cuda")

@@ -25,12 +25,11 @@ def product_lib():
     return capi.product()
 
 
-REFERENCE_LIB = ROOT / "oracle" / "_ref" / "libabpoa_ref.so"      # the unmodified reference, built by oracle/Makefile
-
-
 @pytest.fixture(scope="session")
 def reference_lib():
-    from abpoa_b200 import capi
-    if not REFERENCE_LIB.exists():
-        pytest.skip("oracle/_ref/libabpoa_ref.so not built (reference tree absent and no prebuilt copy)")
-    return capi.load_library(REFERENCE_LIB)
+    """The unmodified reference's answers, stored under tests/golden/ (tests/golden_reference.py); with
+    ABPOA_REFERENCE_RECORD=<file> they come from the live reference and are written to <file>."""
+    from golden_reference import GoldenReference
+    ref = GoldenReference(os.environ.get("ABPOA_REFERENCE_RECORD") or None)
+    yield ref
+    ref.save()

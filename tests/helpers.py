@@ -8,7 +8,6 @@ import numpy as np
 from abpoa_b200.aligner import PoaConfig, PoaSession, encode
 
 INPUTS = Path(__file__).resolve().parent / "golden" / "inputs"
-REFERENCE_LIB = Path(__file__).resolve().parent.parent / "oracle" / "_ref" / "libabpoa_ref.so"
 
 
 def read_fasta(path: Path, m: int = 5) -> list[np.ndarray]:
@@ -35,7 +34,14 @@ def run_group(lib, cfg: PoaConfig, reads, want_msa: bool = True, use_oracle: boo
     use_oracle=True: the graph / consensus / MSA code of `lib` is driven, but every
     alignment comes from the scalar oracle (oracle/libpoa_oracle.so).  That is how the
     CPU-only suite exercises the product's host layer without a GPU -- a test harness
-    arrangement, not a product path."""
+    arrangement, not a product path.
+
+    `lib` may be the stored reference (golden_reference.GoldenReference): the result is then the
+    reference's digest of the same run (compare it with assert_group_equal)."""
+    from golden_reference import GoldenReference
+    if isinstance(lib, GoldenReference):
+        assert not use_oracle and not fast_order
+        return lib.group(cfg, reads, want_msa, weights)
     cfg = PoaConfig(**{**cfg.__dict__, "out_msa": want_msa})
     with PoaSession(cfg, lib) as s:
         if use_oracle:
@@ -71,6 +77,9 @@ def run_group(lib, cfg: PoaConfig, reads, want_msa: bool = True, use_oracle: boo
 
 
 def assert_group_equal(a, b, tag=""):
+    from golden_reference import RefGroup, assert_matches_reference
+    if isinstance(b, RefGroup):
+        return assert_matches_reference(a, b, tag)
     assert len(a["alns"]) == len(b["alns"])
     for i, (x, y) in enumerate(zip(a["alns"], b["alns"])):
         assert x.aligned == y.aligned, f"{tag} read {i}: aligned flag"
@@ -114,27 +123,3 @@ def assert_digest_equal(got, want, tag=""):
         assert x == y, f"{tag} read {i}: {x} != {y}"
     for k in ("cons", "cov_sha1", "msa_len", "msa_sha1"):
         assert got[k] == want[k], f"{tag}: {k} differs"
-
-
-def _ref_records_worker(args):
-    """(spawned process) one group through the unmodified reference: per-read score / CIGAR length /
-    FNV-1a hash of the CIGAR words / DP cells, consensus, coverage."""
-    cfg_kw, reads, want_msa = args
-    from abpoa_b200 import capi
-    from abpoa_b200.batch import fnv1a_words
-    r = run_group(capi.load_library(REFERENCE_LIB), PoaConfig(**cfg_kw), reads, want_msa=want_msa)
-    return {
-        "score": [a.best_score if a.aligned else 0 for a in r["alns"]],
-        "n_cigar": [len(a.cigar) for a in r["alns"]],
-        "hash": [fnv1a_words(a.cigar) if a.aligned else None for a in r["alns"]],
-        "cells": sum(a.cells for a in r["alns"]),
-        "cons": r["cons"], "cov": r["cov"], "msa": r["msa"],
-    }
-
-
-def reference_records(cfg: PoaConfig, groups, want_msa=False, procs=4):
-    """Run the groups through oracle/_ref in parallel worker processes (the reference is single-threaded and,
-    at 10 kbp, page-fault bound: ~15 s per 50-read group)."""
-    import multiprocessing as mp
-    with mp.get_context("spawn").Pool(min(procs, len(groups))) as pool:
-        return pool.map(_ref_records_worker, [(dict(cfg.__dict__), g, want_msa) for g in groups])

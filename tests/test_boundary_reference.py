@@ -1,19 +1,21 @@
-"""Drop-in boundary against the REFERENCE's own files (CPU; skipped where /root/reference does not exist, e.g. on the GPU box):
+"""Drop-in boundary against the REFERENCE's public interface (CPU):
 
-* struct layout: a probe compiled once against /root/reference/include/abpoa.h and once against include/abpoa.h must print the
-  same sizeof / offsetof for every public struct and the same values for every constant;
-* the reference's example programs (example.c, sub_example.c, incre_example.c) compile against OUR header and link against
-  libabpoa_b200.so unchanged (running them needs a GPU; on a GPU box the library's own tests cover the same calls)."""
+* struct layout: a probe compiled against include/abpoa.h must print the same sizeof / offsetof for every public struct and
+  the same values for every constant as the same probe compiled against the reference's abpoa.h (its output is stored in
+  tests/golden/reference_abi.txt);
+* every function of abpoa.h that the reference's example programs (example.c, sub_example.c, incre_example.c) call -- the
+  lists are stored in tests/golden/reference_example_api.json -- is declared by OUR header and exported by
+  libabpoa_b200.so: a program taking the address of each one compiles and links (running the calls needs a GPU; on a GPU
+  box the library's own tests cover them)."""
+import json
 import subprocess
 from pathlib import Path
 
 import pytest
 
 ROOT = Path(__file__).resolve().parent.parent
-REF = Path("/root/reference")
+GOLDEN = Path(__file__).resolve().parent / "golden"
 LIBDIR = ROOT / "abpoa_b200" / "lib"
-
-pytestmark = pytest.mark.skipif(not (REF / "include" / "abpoa.h").exists(), reason="reference tree not present")
 
 PROBE = r'''
 #include <stdio.h>
@@ -57,15 +59,21 @@ def probe(tmp_path, tag, include_dirs):
 
 def test_public_structs_match_the_reference_header(tmp_path):
     ours = probe(tmp_path, "ours", [ROOT / "include"])
-    theirs = probe(tmp_path, "ref", [REF / "include"])
+    theirs = (GOLDEN / "reference_abi.txt").read_text()
     assert ours == theirs, "\n".join(f"{a}   |   {b}" for a, b in zip(ours.splitlines(), theirs.splitlines()) if a != b)
 
 
 @pytest.mark.parametrize("prog", ["example.c", "sub_example.c", "incre_example.c"])
-def test_reference_examples_build_against_this_library(tmp_path, prog):
+def test_reference_example_api_links_against_this_library(tmp_path, prog):
     if not (LIBDIR / "libabpoa_b200.so").exists():
         pytest.skip("library not built")
-    exe = tmp_path / prog.replace(".c", "")
-    r = subprocess.run(["gcc", "-O1", "-w", f"-I{ROOT / 'include'}", "-o", str(exe), str(REF / prog), f"-L{LIBDIR}", "-labpoa_b200", f"-Wl,-rpath,{LIBDIR}", "-lm", "-lz", "-lpthread"],
+    fns = json.loads((GOLDEN / "reference_example_api.json").read_text())[prog]
+    assert fns
+    src = tmp_path / ("uses_" + prog)
+    src.write_text('#include <stdio.h>\n#include "abpoa.h"\nint main(void) {\n'
+                   + "".join(f'    printf("%p\\n", (void *)&{f});\n' for f in fns) + "    return 0;\n}\n")
+    exe = tmp_path / src.stem
+    r = subprocess.run(["gcc", "-O1", "-Wall", "-Werror=implicit-function-declaration", f"-I{ROOT / 'include'}", "-o", str(exe), str(src),
+                        f"-L{LIBDIR}", "-labpoa_b200", f"-Wl,-rpath,{LIBDIR}", "-Wl,--no-undefined", "-lm", "-lz", "-lpthread"],
                        capture_output=True, text=True)
     assert r.returncode == 0, r.stderr

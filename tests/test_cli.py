@@ -3,7 +3,7 @@
 CPU part: the reader (poa_read_fastx, grammar of the reference's kseq-based abpoa_read_seq) on the reference's own
 test inputs, plain and gzip-compressed.  GPU part: the real binary reproduces the md5 vectors recorded from the
 reference CLI (SURVEY 8c / tests/golden/golden.json) and, in list mode (-l: all files as ONE GPU batch), prints
-byte for byte what the reference binary prints for the same list."""
+byte for byte what the reference binary prints for the same list (md5 stored, tests/golden_reference.py)."""
 import ctypes as C
 import gzip
 import hashlib
@@ -19,7 +19,7 @@ from helpers import INPUTS
 
 ROOT = Path(__file__).resolve().parent.parent
 BIN = ROOT / "abpoa_b200" / "bin" / "abpoa"
-REF_BIN = ROOT / "oracle" / "_ref" / "abpoa_ref"
+REF_BIN = ROOT / "oracle" / "_ref" / "abpoa_ref"      # the reference CLI (oracle/Makefile), only to record the stored md5
 
 
 def read_with_library(lib, path):
@@ -102,21 +102,23 @@ def test_cli_md5_vector_test_fa():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("opts", [[], ["-r1"], ["-r2"], ["-r5"], ["-m", "1", "-r2"], ["-Q", "-r2"]])
-def test_cli_list_mode_matches_reference_binary(tmp_path, opts):
+def test_cli_list_mode_matches_reference_binary(reference_lib, tmp_path, opts):
     """-l: every file is one read group; ours runs them as one GPU batch (device chain for consensus output, launch
-    engine otherwise) and must print what the reference prints file by file."""
-    if not REF_BIN.exists():
-        pytest.skip("oracle/_ref/abpoa_ref not built")
+    engine otherwise) and must print what the reference prints file by file.  The files are named relative to the
+    working directory, so the list and the output are the same wherever the test runs."""
     files = []
     for g in range(7):
         reads = synth.make_group(7000 + g, 4 + g % 4, 150 + 60 * g, 0.06)
         p = tmp_path / f"g{g}.fa"
         p.write_text("".join(f">read{g}_{i} len={len(r)}\n{decode(r)}\n" for i, r in enumerate(reads)))
-        files.append(p)
-    files.append(INPUTS / "seq.fa")
-    files.append(INPUTS / "heter.fq")
+        files.append(p.name)
+    for f in ("seq.fa", "heter.fq"):
+        (tmp_path / f).write_bytes((INPUTS / f).read_bytes())
+        files.append(f)
     lst = tmp_path / "list.txt"
     lst.write_text("".join(f"{p}\n" for p in files))
-    ours = subprocess.run([str(BIN), *opts, "-l", str(lst)], capture_output=True, check=True).stdout
-    ref = subprocess.run([str(REF_BIN), *opts, "-l", str(lst)], capture_output=True, check=True).stdout
-    assert ours == ref
+    run = lambda exe: subprocess.run([str(exe), *opts, "-l", lst.name], cwd=tmp_path, capture_output=True, check=True).stdout
+    ours = run(BIN)
+    question = (opts, [(tmp_path / f).read_bytes().decode() for f in files])
+    ref = reference_lib.value("cli_list_md5", question, lambda lib: hashlib.md5(run(REF_BIN)).hexdigest())
+    assert hashlib.md5(ours).hexdigest() == ref

@@ -2,14 +2,14 @@
 must give, group by group, exactly what the reference gives for abpoa_msa() on that group --
 per-read best score, CIGAR length and FNV hash of the CIGAR words, DP cells, consensus,
 coverage and RC-MSA."""
-import numpy as np
 import pytest
 
 from abpoa_b200 import synth
 from abpoa_b200.aligner import PoaConfig
-from abpoa_b200.batch import BatchEngine, fnv1a_words
+from abpoa_b200.batch import BatchEngine
 from cases import AFFINE, LINEAR
 from abpoa_b200.capi import ABPOA_LOCAL_MODE
+from golden_reference import assert_batch_matches_reference
 from helpers import run_group
 
 pytestmark = pytest.mark.gpu
@@ -22,16 +22,7 @@ def check_batch(reference_lib, cfg, groups, **engine_kw):
     assert st["alignments"] == sum(max(len(g) - 1, 0) for g in groups)
     for gi, (g, r) in enumerate(zip(groups, got)):
         ref = run_group(reference_lib, cfg, g, want_msa=cfg.out_msa)
-        assert r.dp_cells == sum(a.cells for a in ref["alns"]), f"group {gi}: cells"
-        for i, a in enumerate(ref["alns"]):
-            if not a.aligned:
-                continue
-            assert r.read_best_score[i] == a.best_score, f"group {gi} read {i}: score"
-            assert r.read_n_cigar[i] == len(a.cigar), f"group {gi} read {i}: n_cigar"
-            assert int(r.read_cigar_hash[i]) == fnv1a_words(a.cigar), f"group {gi} read {i}: cigar hash"
-        assert len(r.cons) == len(ref["cons"]) and all(np.array_equal(x, y) for x, y in zip(r.cons, ref["cons"])), f"group {gi}: consensus"
-        assert all(np.array_equal(x, y) for x, y in zip(r.cov, ref["cov"])), f"group {gi}: coverage"
-        assert len(r.msa) == len(ref["msa"]) and all(np.array_equal(x, y) for x, y in zip(r.msa, ref["msa"])), f"group {gi}: msa"
+        assert_batch_matches_reference(r, ref, f"group {gi}")
 
 
 def test_batch_affine_many_groups(reference_lib):

@@ -3,7 +3,7 @@
 * single-alignment path (abpoa.h: abpoa_align_sequence_to_graph + abpoa_add_graph_alignment) against
   the golden vectors generated from the unmodified reference (tests/golden/golden.json) -- no oracle,
   no reference library involved: per-read score, CIGAR sha1, end points, DP cells, consensus, RC-MSA;
-* batch engine (abpoa_gpu.h) against the live reference (oracle/_ref) with per-read CIGAR hashes;
+* batch engine (abpoa_gpu.h) against the reference's stored answers (tests/golden_reference.py) with per-read CIGAR hashes;
 * every fallback of the launcher forced through environment switches: generic int16 kernel
   (ABPOA_GPU_NO_P16), range guard of the packed kernel (ABPOA_GPU_FORCE_P16 on a case that needs 32
   bits), plane-slab overflow redo (ABPOA_GPU_SLAB_PCT), Kahn order instead of the spliced order
@@ -20,9 +20,10 @@ import pytest
 
 from abpoa_b200 import capi, synth
 from abpoa_b200.aligner import PoaConfig, PoaSession
-from abpoa_b200.batch import BatchEngine, fnv1a_words
+from abpoa_b200.batch import BatchEngine
 from abpoa_b200.capi import abpoa_res_t, c_u8_p
 from cases import AFFINE, CASES, case_reads, case_weights
+from golden_reference import GoldenReference, arrays_digest, assert_batch_matches_reference, digest
 from helpers import assert_digest_equal, assert_group_equal, group_digest, run_group
 
 pytestmark = pytest.mark.gpu
@@ -103,17 +104,7 @@ def check_batch(reference_lib, cfg, groups, weights=None, cells=True, **engine_k
     assert st["alignments"] >= sum(max(len(g) - 1, 0) for g in groups)
     for gi, (g, r) in enumerate(zip(groups, got)):
         ref = run_group(reference_lib, cfg, g, want_msa=cfg.out_msa, weights=weights[gi] if weights else None)
-        if cells:
-            assert r.dp_cells == sum(a.cells for a in ref["alns"]), f"group {gi}: cells"
-        for i, a in enumerate(ref["alns"]):
-            if not a.aligned:
-                continue
-            assert r.read_best_score[i] == a.best_score, f"group {gi} read {i}: score"
-            assert r.read_n_cigar[i] == len(a.cigar), f"group {gi} read {i}: n_cigar"
-            assert int(r.read_cigar_hash[i]) == fnv1a_words(a.cigar), f"group {gi} read {i}: cigar hash"
-        assert len(r.cons) == len(ref["cons"]) and all(np.array_equal(x, y) for x, y in zip(r.cons, ref["cons"])), f"group {gi}: consensus"
-        assert all(np.array_equal(x, y) for x, y in zip(r.cov, ref["cov"])), f"group {gi}: coverage"
-        assert len(r.msa) == len(ref["msa"]) and all(np.array_equal(x, y) for x, y in zip(r.msa, ref["msa"])), f"group {gi}: msa"
+        assert_batch_matches_reference(r, ref, f"group {gi}", cells=cells)
     return st
 
 
@@ -170,10 +161,13 @@ def test_more_than_32_predecessors(product_lib, reference_lib, gap):
     cfg = PoaConfig(**(AFFINE if gap == "affine" else {}))
     reads = deletion_fan()
     ref = run_group(reference_lib, cfg, reads)
-    with PoaSession(cfg, reference_lib) as s:
-        s.run_reads(reads, count_cells=False)
-        g = s.ab.contents.abg.contents
-        deg = max(g.node[i].in_edge_n for i in range(g.node_n))
+
+    def max_in_degree(lib):
+        with PoaSession(cfg, lib) as s:
+            s.run_reads(reads, count_cells=False)
+            g = s.ab.contents.abg.contents
+            return max(g.node[i].in_edge_n for i in range(g.node_n))
+    deg = reference_lib.value("max_in_degree", (cfg.__dict__, reads), max_in_degree)
     assert deg > 32, f"the construction only reached in-degree {deg}"
     assert_group_equal(run_group(product_lib, cfg, reads), ref, f"fan/{gap}")
 
@@ -195,11 +189,17 @@ def strand_mix(seed, n, length):
 
 
 def msa_whole(lib, cfg, reads):
-    with PoaSession(cfg, lib) as s:
-        s.msa(reads)
-        abs_ = s.ab.contents.abs.contents
-        is_rc = [int(abs_.is_rc[i]) for i in range(len(reads))]
-        return {"cons": s.consensus(), "cov": s.consensus_cov(), "msa": s.msa_rows(), "is_rc": is_rc}
+    """abpoa_msa over the whole group: which reads were flipped, digests of consensus, coverage and RC-MSA
+    (for the stored reference: its stored answer)."""
+    def run(lib):
+        with PoaSession(cfg, lib) as s:
+            s.msa(reads)
+            abs_ = s.ab.contents.abs.contents
+            is_rc = [int(abs_.is_rc[i]) for i in range(len(reads))]
+            return {"cons": arrays_digest(s.consensus()), "cov": arrays_digest(s.consensus_cov()), "msa": arrays_digest(s.msa_rows()), "is_rc": is_rc}
+    if isinstance(lib, GoldenReference):
+        return lib.value("msa_whole", (cfg.__dict__, reads), run)
+    return run(lib)
 
 
 def test_amb_strand_msa(product_lib, reference_lib):
@@ -209,8 +209,8 @@ def test_amb_strand_msa(product_lib, reference_lib):
     a, b = msa_whole(product_lib, cfg, reads), msa_whole(reference_lib, cfg, reads)
     assert sum(b["is_rc"]) >= 2, "the reference flipped no read: the case does not exercise -s"
     assert a["is_rc"] == b["is_rc"]
-    assert all(np.array_equal(x, y) for x, y in zip(a["cons"], b["cons"]))
-    assert len(a["msa"]) == len(b["msa"]) and all(np.array_equal(x, y) for x, y in zip(a["msa"], b["msa"]))
+    assert a["cons"] == b["cons"]
+    assert a["msa"] == b["msa"]
 
 
 def test_amb_strand_batch(product_lib, reference_lib):
@@ -220,13 +220,17 @@ def test_amb_strand_batch(product_lib, reference_lib):
         got = eng.run(cfg, groups)
     for gi, (g, r) in enumerate(zip(groups, got)):
         ref = msa_whole(reference_lib, cfg, g)
-        assert all(np.array_equal(x, y) for x, y in zip(r.cons, ref["cons"])), f"group {gi}: consensus"
-        assert len(r.msa) == len(ref["msa"]) and all(np.array_equal(x, y) for x, y in zip(r.msa, ref["msa"])), f"group {gi}: msa"
+        assert arrays_digest(r.cons) == ref["cons"], f"group {gi}: consensus"
+        assert arrays_digest(r.msa) == ref["msa"], f"group {gi}: msa"
 
 
 def subgraph_walk(lib, cfg, reads, windows):
     """The loop of the reference's sub_example.c: read i is aligned to the sub-graph between the nodes
-    that enclose [inc_beg, inc_end] (abpoa_subgraph_nodes) and fused with abpoa_add_subgraph_alignment."""
+    that enclose [inc_beg, inc_end] (abpoa_subgraph_nodes) and fused with abpoa_add_subgraph_alignment.
+    Per read (rc, window begin, window end, score, digest of the graph-CIGAR, end points), digests of the
+    consensus and the RC-MSA (for the stored reference: its stored answer)."""
+    if isinstance(lib, GoldenReference):
+        return lib.value("subgraph_walk", (cfg.__dict__, reads, windows), lambda live: subgraph_walk(live, cfg, reads, windows))
     d = lib.dll
     d.abpoa_subgraph_nodes.argtypes = [capi.abpoa_t_p, capi.abpoa_para_t_p, C.c_int, C.c_int, capi.c_int_p, capi.c_int_p]
     d.abpoa_align_sequence_to_subgraph.restype = C.c_int
@@ -245,12 +249,12 @@ def subgraph_walk(lib, cfg, reads, windows):
                 d.abpoa_subgraph_nodes(s.ab, s.abpt, wb, we, C.byref(eb), C.byref(ee))
             rc = d.abpoa_align_sequence_to_subgraph(s.ab, s.abpt, eb.value, ee.value, r.ctypes.data_as(c_u8_p), len(r), C.byref(res))
             cig = np.ctypeslib.as_array(res.graph_cigar, shape=(res.n_cigar,)).copy() if res.n_cigar > 0 else np.zeros(0, dtype=np.uint64)
-            out.append((rc, eb.value, ee.value, int(res.best_score) if rc >= 0 else 0, cig, (res.node_s, res.node_e, res.query_s, res.query_e) if rc >= 0 else None))
+            out.append([rc, eb.value, ee.value, int(res.best_score) if rc >= 0 else 0, digest(cig), [res.node_s, res.node_e, res.query_s, res.query_e] if rc >= 0 else None])
             d.abpoa_add_subgraph_alignment(s.ab, s.abpt, eb.value, ee.value, r.ctypes.data_as(c_u8_p), None, len(r), None, res, i, len(reads), 0)
             if res.n_cigar > 0:
                 capi.libc_free(res.graph_cigar)
         s.generate()
-        return out, s.consensus(), s.msa_rows()
+        return [out, arrays_digest(s.consensus()), arrays_digest(s.msa_rows())]
 
 
 @pytest.mark.parametrize("path_score", [False, True])
@@ -271,12 +275,13 @@ def test_subgraph_alignment(product_lib, reference_lib, path_score):
     cfg = PoaConfig(inc_path_score=path_score, out_msa=True)
     a = subgraph_walk(product_lib, cfg, reads, windows)
     b = subgraph_walk(reference_lib, cfg, reads, windows)
+    assert len(a[0]) == len(b[0])
     for i, (x, y) in enumerate(zip(a[0], b[0])):
         assert x[:4] == y[:4], f"read {i}: rc / window / score {x[:4]} vs {y[:4]}"
-        assert np.array_equal(x[4], y[4]), f"read {i}: graph-CIGAR"
+        assert x[4] == y[4], f"read {i}: graph-CIGAR"
         assert x[5] == y[5], f"read {i}: ends"
-    assert all(np.array_equal(x, y) for x, y in zip(a[1], b[1]))
-    assert len(a[2]) == len(b[2]) and all(np.array_equal(x, y) for x, y in zip(a[2], b[2]))
+    assert a[1] == b[1]
+    assert a[2] == b[2]
 
 
 # ------------------------------------------------------------------------------------------- a7: banded linear gaps, lane-exact

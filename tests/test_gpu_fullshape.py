@@ -1,32 +1,24 @@
 """GPU parity at the BENCHMARKED sizes (BASELINE.json configs 2-5), product vs the unmodified
-reference (oracle/_ref): per-read best score, graph-CIGAR length and FNV-1a hash of every CIGAR word,
+reference (its stored answers, tests/golden_reference.py): per-read best score, graph-CIGAR length and FNV-1a hash of every CIGAR word,
 DP-cell totals, consensus and coverage.
 
 Small cases cannot reach what these do: 25 k-row graphs, bands wider than one 256-cell pass, scores
 close to the packed kernel's int16 window, graphs past the point where the reference itself switches
 to int32 (gn > 16 364), 20-pass rows in local mode.
 """
-import numpy as np
 import pytest
 
 from abpoa_b200 import synth
 from abpoa_b200.batch import BatchEngine
-from helpers import reference_records
+from golden_reference import assert_batch_matches_reference
 
 pytestmark = pytest.mark.gpu
 
 
 def compare(got, ref, tag):
+    assert len(got) == len(ref)
     for gi, (r, w) in enumerate(zip(got, ref)):
-        assert r.dp_cells == w["cells"], f"{tag} group {gi}: DP cells {r.dp_cells} != {w['cells']}"
-        for i in range(len(w["score"])):
-            if w["hash"][i] is None:
-                continue
-            assert r.read_best_score[i] == w["score"][i], f"{tag} group {gi} read {i}: score"
-            assert r.read_n_cigar[i] == w["n_cigar"][i], f"{tag} group {gi} read {i}: n_cigar"
-            assert int(r.read_cigar_hash[i]) == w["hash"][i], f"{tag} group {gi} read {i}: CIGAR hash"
-        assert len(r.cons) == len(w["cons"]) and all(np.array_equal(x, y) for x, y in zip(r.cons, w["cons"])), f"{tag} group {gi}: consensus"
-        assert all(np.array_equal(x, y) for x, y in zip(r.cov, w["cov"])), f"{tag} group {gi}: coverage"
+        assert_batch_matches_reference(r, w, f"{tag} group {gi}", msa=False)
 
 
 @pytest.mark.parametrize("engine", ["chain", "launch"])
@@ -37,7 +29,7 @@ def test_full_shape(reference_lib, name, n_groups, engine):
     if engine == "chain" and w.cfg.align_mode != 0:
         pytest.skip("local mode always takes the launch engine")
     groups = w.groups(n_groups, base_seed=4200)
-    ref = reference_records(w.cfg, groups)
+    ref = reference_lib.groups(w.cfg, groups)
     with BatchEngine() as eng:
         got = eng.run(w.cfg, groups, record_reads=True, no_chain=(engine == "launch"))
         st = eng.stats()
@@ -52,7 +44,7 @@ def test_full_shape_convex_generic_kernels(reference_lib, monkeypatch):
     monkeypatch.setenv("ABPOA_GPU_NO_P16", "1")
     w = synth.WORKLOADS["convex_10k"]
     groups = w.groups(1, base_seed=4300)
-    ref = reference_records(w.cfg, groups)
+    ref = reference_lib.groups(w.cfg, groups)
     with BatchEngine(n_workers=1, groups_per_launch=1) as eng:
         got = eng.run(w.cfg, groups, record_reads=True)
     compare(got, ref, "convex_10k/generic")
